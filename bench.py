@@ -6,7 +6,7 @@ One step = one pass of the hot path over one synthetic ComplexF32 stream shard:
     P = welch_pgram(y[:2^26])   n = nfft = 4096, 50 % overlap, hanning, two-sided            (Welch stage of the metric)
 metric = input samples per second through both stages (Gsamples/s), whole job over all ranks.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--log2n 26] [--workload ...]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--log2n 26] [--workload ...] [--dump-outputs DIR]
   N > 1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N
 
 Multi-GPU (the contract line is weak scaling): every rank owns a 2^26-sample shard of one long stream (plus the nv-1
@@ -99,6 +99,33 @@ class ClockSampler:
                     reasons.add(nme)
         return {"sm_mhz": float(np.median(sm)) if sm else None, "sm_max_mhz": max(smax) if smax else None,
                 "samples": len(sm), "reasons": sorted(reasons)}
+
+
+DUMP_SAMPLE, DUMP_EDGE, DUMP_SEED = 1 << 20, 4096, 20260101
+
+
+def dump_outputs(out_dir, arrays, d):
+    """--dump-outputs: write each array the timed path handed back in its last step as <out_dir>/<name>.npy, so that two
+    builds run with the same arguments (same seeded inputs) can be compared output for output.  Complex arrays are written
+    as float (re, im) pairs along a trailing axis of 2.  An array of more than DUMP_SAMPLE elements is written as a fixed
+    sample of its flattened elements -- the first and last DUMP_EDGE plus DUMP_SAMPLE drawn with a fixed seed -- and the
+    sampled flat indices go beside it as <name>_index.npy (float64, exact); about 16 MB per sampled array.  With several
+    ranks every rank writes its own arrays, suffixed _rank<r>."""
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    suffix = f"_rank{d.rank}" if d.world > 1 else ""
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            n = t.numel()
+            rng = np.random.default_rng(DUMP_SEED)
+            idx = np.unique(np.concatenate([np.arange(DUMP_EDGE), np.arange(n - DUMP_EDGE, n), rng.integers(0, n, DUMP_SAMPLE)]))
+            t = t.reshape(-1)[torch.from_numpy(idx).to(t.device)]
+            np.save(os.path.join(out_dir, f"{name}{suffix}_index.npy"), idx.astype(np.float64))
+        t = t.cpu()
+        a = (torch.view_as_real(t) if t.is_complex() else t).numpy()
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(out_dir, f"{name}{suffix}.npy"), a)
 
 
 def measured_peak_gbs():
@@ -283,6 +310,7 @@ class Dist:
         if not torch.cuda.is_available():
             raise SystemExit("bench.py --impl ours needs a CUDA device (no CPU fallback)")
         torch.cuda.set_device(self.local_rank)
+        torch.manual_seed(1000 + self.rank)            # same inputs every run, so --dump-outputs can compare two builds
         from dspb200 import _lib
         _lib.check(_lib.lib.dspb200_set_device(self.local_rank))
         self.dev = torch.device("cuda", self.local_rank)
@@ -609,6 +637,8 @@ def run_ours(args):
     if rank == 0:
         clocks.start()
     res = cw.time(args.steps, args.warmup)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"conv_out": cw.y, "welch_psd": cw.last}, d)
     chk = cw.check() if not args.no_check else None
 
     e2e = e2e_serial = e2e_host = None
@@ -733,6 +763,7 @@ def run_other_workload(args):
         k = (length - nn) // (nn - nov) + 1
         out = torch.empty((nn // 2 + 1) * k * (c1 - c0), device=dev, dtype=torch.float32)
         fn = lambda: plan.stft_dev(x.data_ptr(), length, c1 - c0, float(nn), True, out.data_ptr(), sp)   # noqa: E731
+        outputs = {"spectrogram_power": out}
         units, unit = nchan * length, "Gsamples/s"
         bytes_local = 4.0 * (c1 - c0) * length + 4.0 * out.numel()
         desc = f"spectrogram 64 ch x 2^22 Float32, n = nfft = 1024, noverlap = 768 (BASELINE configs[3]); channels {c0}..{c1 - 1} on rank 0"
@@ -762,6 +793,7 @@ def run_other_workload(args):
             fn = lambda: plan.exec_dev(x.data_ptr(), length, c1 - c0, y.data_ptr(), sp)   # noqa: E731
         else:
             fn = lambda: plan.exec_dev(x.data_ptr(), length, c1 - c0, y.data_ptr(), length, sp)   # noqa: E731
+        outputs = {"filt_out": y}
         units, unit = ncol * length, "Gsamples/s"
         bytes_local = 8.0 * (c1 - c0) * length
         desc = (f"filt(b, 1, x) 257-tap FIR on a 2^20 x 64 Float32 matrix (BASELINE configs[0], 64 columns), "
@@ -798,6 +830,7 @@ def run_other_workload(args):
         plan = _lib.ResamplePlan(np.complex64, h, 3, 2)
         y = torch.empty(sh.out_count, device=dev, dtype=torch.complex64)
         fn = lambda: plan.exec_range_dev(x.data_ptr(), sh.in_begin, nx_local, n0, phi0, y.data_ptr(), sh.j_begin, sh.out_count, sp)   # noqa: E731
+        outputs = {"resample_out": y}
 
         def check():
             # both ends of this rank's output range (the shard boundaries) against the polyphase sum in Float64
@@ -834,6 +867,7 @@ def run_other_workload(args):
             plan.welch_dev(x.data_ptr(), n, r, pw.data_ptr(), sp)
             if d.pg is not None:
                 d.pg.all_reduce(pw)
+        outputs = {"welch_psd": pw}
         units, unit = n * world, "Gsamples/s"
         bytes_local = 4.0 * n
         desc = f"welch_pgram 2^{args.log2n} Float32 per GPU, n = nfft = 4096, 50 % overlap, hanning (BASELINE configs[2]); PSD all-reduce"
@@ -866,6 +900,8 @@ def run_other_workload(args):
     ms = d.max_over_ranks([a.elapsed_time(b) / args.steps])[0]
     launches = _lib.launch_count() - l0
     clk = clocks.stop() if rank == 0 else None
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs, d)
     chk = None
     if not args.no_check:
         err, tol_, what = check()
@@ -901,7 +937,13 @@ def main():
     ap.add_argument("--no-check", action="store_true")
     ap.add_argument("--no-strong", action="store_true")
     ap.add_argument("--graph", action="store_true", help="also time the strong-scaling step replayed from one CUDA graph")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last step as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:
