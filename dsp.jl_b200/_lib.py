@@ -9,7 +9,7 @@ import os
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-LIB_PATH = os.environ.get("DSPB200_LIB") or os.path.join(_HERE, "libdspb200.so")   # DSPB200_LIB: alternative build (A/B tests)
+LIB_PATH = os.environ.get("DSPB200_LIB") or os.path.join(_HERE, "libdspb200.so")   # DSPB200_LIB: another build, e.g. to compare two builds output for output
 
 F32, F64, C32, C64 = 0, 1, 2, 3
 _NP2DT = {np.dtype(np.float32): F32, np.dtype(np.float64): F64, np.dtype(np.complex64): C32, np.dtype(np.complex128): C64}

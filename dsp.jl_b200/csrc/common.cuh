@@ -33,39 +33,6 @@ template <typename T> __host__ __device__ __forceinline__ cx<T> mul_mi(cx<T> a) 
 template <typename T> __host__ __device__ __forceinline__ T cabs2(cx<T> a) { return a.x * a.x + a.y * a.y; }
 
 // ----------------------------------------------------------------------------------------------
-// Blackwell packed FP32x2 (sm_100: FADD2 / FMUL2 / FFMA2).  A ComplexF32 value is exactly one f32x2 operand, and the
-// SASS operand modifiers cover complex arithmetic for free: per-half negation, half swap (LO_HI) -- i.e. multiply by
-// +-i -- and scalar broadcast (.F32).  So on the device
-//     a +- b          = 1 FADD2                      (2 scalar ops)
-//     a +- (+-i) b    = 1 FADD2 with LO_HI / NP      (2)
-//     a * w (complex) = FMUL2 + FFMA2                (4: 2 FMUL + 2 FFMA)
-// which halves the FP32 issue slots of every butterfly (measured on B200: FADD2 sustains the scalar FADD lane rate,
-// FFMA2 1.5x the three-register scalar FFMA rate, profiles/microbench/f32x2.cu).  Host builds use the scalar forms.
-// A/B on B200 (profiles/README.md): the FFT kernels are bound by the shared-memory pipe and barrier phases, not by FP32
-// issue, so halving the FP instruction count moves the kernel times by only -3 % .. +5 %; the packed path is therefore
-// opt-in (-DDSP_USE_F32X2) and the default build keeps the scalar forms.
-#if defined(__CUDA_ARCH__) && (__CUDA_ARCH__ >= 1000) && defined(DSP_USE_F32X2)
-#define DSP_F32X2 1
-__device__ __forceinline__ cx<float> operator+(cx<float> a, cx<float> b) {
-    const float2 r = __fadd2_rn(make_float2(a.x, a.y), make_float2(b.x, b.y));
-    return mkc<float>(r.x, r.y);
-}
-__device__ __forceinline__ cx<float> operator-(cx<float> a, cx<float> b) {
-    const float2 r = __fadd2_rn(make_float2(a.x, a.y), make_float2(-b.x, -b.y));
-    return mkc<float>(r.x, r.y);
-}
-__device__ __forceinline__ cx<float> cmul(cx<float> a, cx<float> b) {
-    const float2 t = __fmul2_rn(make_float2(a.y, a.y), make_float2(-b.y, b.x));
-    const float2 r = __ffma2_rn(make_float2(a.x, a.x), make_float2(b.x, b.y), t);
-    return mkc<float>(r.x, r.y);
-}
-__device__ __forceinline__ cx<float> cscale(cx<float> a, float s) {
-    const float2 r = __fmul2_rn(make_float2(a.x, a.y), make_float2(s, s));
-    return mkc<float>(r.x, r.y);
-}
-#endif
-
-// ----------------------------------------------------------------------------------------------
 // dtype traits
 template <typename E> struct elt_traits;
 template <> struct elt_traits<float>       { using real = float;  static constexpr bool is_cplx = false; };
@@ -163,8 +130,7 @@ static inline int64_t cdiv(int64_t a, int64_t b) { return (a + b - 1) / b; }
 // in `pdl_wait()` until the previous grid has completed and its memory is visible -- the launch gap and the table prologue
 // (68 KB per CTA for the 16384-point kernel) overlap the previous kernel's tail instead of following it.  EVERY thread
 // executes pdl_wait() before its first access to anything a preceding kernel could have written or still be reading, so
-// the chain is transitive.  Without the launch attribute both instructions are no-ops.  DSPB200_PDL=0 turns it off.
-bool pdl_enabled();
+// the chain is transitive.  Without the launch attribute both instructions are no-ops.
 #ifdef __CUDACC__
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
 __device__ __forceinline__ void pdl_launch_dependents() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
@@ -177,7 +143,7 @@ static inline cudaError_t launch_pdl(void (*kern)(KA...), unsigned grid, unsigne
     cfg.stream = st;
     cudaLaunchAttribute at[1];
     at[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    at[0].val.programmaticStreamSerializationAllowed = pdl_enabled() ? 1 : 0;
+    at[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = at;
     cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kern, KA(args)...);

@@ -19,20 +19,6 @@
 #include "common.cuh"
 #include <math.h>
 
-// wave-gated shared-memory loads after CTA-wide barriers (see fft_gate_wait); 0 switches it off for A/B timing
-#ifndef DSP_FFT_GATE
-#define DSP_FFT_GATE 1
-#endif
-// timing probes (wrong results, never in the shipped library): bit 0 skips the stride-256 passes, bit 1 replaces the
-// first-pass global loads by constants, bit 2 the H loads, bit 3 drops the global stores, bit 4 skips the stride-16 passes
-#ifndef DSP_PROBE
-#define DSP_PROBE 0
-#endif
-// last-pass twiddle table of the 512- / 1024- / 2048-point Float32 transforms in shared memory (1) or global memory via L1 (0)
-#ifndef DSP_TL_SMEM_SMALL
-#define DSP_TL_SMEM_SMALL 1
-#endif
-
 namespace dspb200 {
 
 // ---------------------------------------------------------------------------------------------- layout
@@ -238,7 +224,7 @@ template <typename T> struct FftCtx {
 
 template <typename T, int N> __host__ __device__ constexpr bool fft_tl_in_smem() {
     // 16384: W_N^t alone, 32 KB; 512 / 1024 / 2048: the whole last-pass table, 2 / 4 / 8 KB (several CTAs per SM still fit)
-    return sizeof(T) == 4 && (N == 16384 || DSP_TL_SMEM_SMALL && (N == 512 || N == 1024 || N == 2048));
+    return sizeof(T) == 4 && (N == 16384 || N == 512 || N == 1024 || N == 2048);
 }
 template <int N> __host__ __device__ constexpr int fft_tl_len() { return (N / fft_plan_traits<N>::RL) * fft_plan_traits<N>::TLK; }
 template <int N> __host__ __device__ constexpr bool fft_uses_t16() { return N >= 256; }
@@ -419,22 +405,6 @@ __host__ __device__ __forceinline__ void fft_first_pass(const FftCtx<T>& c, int 
     }
 }
 
-// First pass on operands that are already in registers (v[it][r] = sample tid + it NT + r N/16): the overlap-save kernel
-// loads the next unit's samples before the previous unit's last pass, so the L2 -> SM transfer overlaps that pass.
-template <typename T, int N, int NT, bool SYNC, int ITERS, class Scope = FftCtaScope>
-__device__ __forceinline__ void fft_first_pass_regs(const FftCtx<T>& c, int tid, cx<T> (&v)[ITERS][16], Scope sc = Scope()) {
-    constexpr int Q = fft_plan_traits<N>::Q;
-    static_assert(ITERS == (Q + NT - 1) / NT, "register tile does not match the thread count");
-#pragma unroll
-    for (int it = 0; it < ITERS; ++it) {
-        const int b = tid + it * NT;
-        const bool active = (Q % NT == 0) || b < Q;
-        if (active) fft_bfly16_plain<T>(v[it]);
-        if constexpr (SYNC) { if (it == 0) sc.sync(); }
-        if (active) fft_store_block<T, N>(c.sm, b, v[it]);
-    }
-}
-
 // Twiddled radix-16 pass at stride S (16 or 256), in place.
 template <typename T, int N, int NT, int S, bool GATE = false>
 __host__ __device__ __forceinline__ void fft_pass16(const FftCtx<T>& c, int tid) {
@@ -492,14 +462,10 @@ __device__ __forceinline__ void fft_middle(const FftCtx<T>& c, int tid, Scope sc
     constexpr int NMID = fft_plan_traits<N>::NMID;
     static_assert(NMID < 2 || std::is_same<Scope, FftCtaScope>::value, "thread groups run transforms of at most 4096 points");
     if constexpr (NMID >= 1) {
-#if !(DSP_PROBE & 16)
-        fft_pass16<T, N, NT, 16, DSP_FFT_GATE != 0>(c, tid);
-#endif
+        fft_pass16<T, N, NT, 16, true>(c, tid);
         if constexpr (NMID == 2) {
             fft_group256_sync<NT>(tid);
-#if !(DSP_PROBE & 1)
             fft_pass16<T, N, NT, 256>(c, tid);
-#endif
         }
         sc.sync();
     }

@@ -53,45 +53,28 @@ template <typename T> __host__ __device__ __forceinline__ void store_block(cx<T>
     for (int r = 0; r < 32; r += 2) sts2<T>(p + pad(r), v[r], v[r + 1]);
 }
 
-// Load gating (fft_core.cuh, fft_gate_wait / fft_gate_open): GATE bit 0 = wait for the previous 256-thread wave before the
-// loads, bit 1 = let the next wave go after them.  Only after CTA-wide barriers, each wave through each gate exactly once.
-template <int GATE> __device__ __forceinline__ void gate_in(int tid) {
-#ifdef __CUDA_ARCH__
-    if constexpr ((GATE & 1) && DSP_FFT_GATE) fft_gate_wait<NT>(tid);
-#endif
-}
-template <int GATE> __device__ __forceinline__ void gate_out(int tid) {
-#ifdef __CUDA_ARCH__
-    if constexpr ((GATE & 2) && DSP_FFT_GATE) fft_gate_open<NT>(tid);
-#endif
-}
-
 // middle pass: radix 32 at stride 32, butterfly b = (blk, t): slots blk*1024 + t + 32 r
-template <typename T, int GATE = 0> __host__ __device__ __forceinline__ void middle_pass(const Ctx<T>& c, int tid) {
+template <typename T> __host__ __device__ __forceinline__ void middle_pass(const Ctx<T>& c, int tid) {
     const int t = tid & 31;
     cx<T>* p = c.sm + pad((tid >> 5) * 1024 + t);
     cx<T> v[32], w[16];
-    gate_in<GATE>(tid);
 #pragma unroll
     for (int i = 0; i < 16; i += 2) lds2<T>(c.t32 + ((i >> 1) * 32 + t) * 2, w[i], w[i + 1]);
 #pragma unroll
     for (int r = 0; r < 32; ++r) v[r] = p[pad(32 * r)];
-    gate_out<GATE>(tid);
     fft_bfly<T, 32, false>(v, w);
 #pragma unroll
     for (int r = 0; r < 32; ++r) p[pad(32 * r)] = v[r];
 }
 
 // last pass of thread unit tp < 1024: v[r] = X[tp + 1024 r]
-template <typename T, int GATE = 0> __host__ __device__ __forceinline__ void last_pass(const Ctx<T>& c, int tp, cx<T> (&v)[16], int tid = 0) {
+template <typename T> __host__ __device__ __forceinline__ void last_pass(const Ctx<T>& c, int tp, cx<T> (&v)[16]) {
     const cx<T>* p = c.sm + pad(tp);
     cx<T> w[8];
-    gate_in<GATE>(tid);
 #pragma unroll
     for (int i = 0; i < 8; i += 2) lds2<T>(c.t1024 + ((i >> 1) * 1024 + tp) * 2, w[i], w[i + 1]);
 #pragma unroll
     for (int r = 0; r < 16; ++r) v[r] = p[pad(1024 * r)];
-    gate_out<GATE>(tid);
     fft_bfly<T, 16, false>(v, w);
 }
 

@@ -5,75 +5,17 @@
 //     y[i] = fma(x[i], b[1], fma(x[i-1], b[2], ... fma(x[i-nb+2], b[nb-1], x[i-nb+1]*b[nb])))
 // i.e. one fused multiply-add per tap, oldest tap first.  This kernel evaluates exactly that chain per
 // output, so Float32/Float64 results match the reference bit for bit on FMA hardware.
-// Two kernels evaluate it: fir_tile_kernel (default; fir_tile.cuh: 8 outputs per thread, 8 taps per chunk, 128-bit loads,
-// 62-69 % of the FP32 peak) and the round-1 fir_td_kernel below (CTA = 256 threads x 4 consecutive outputs, one tap per
-// iteration; kept as the A/B baseline behind DSPB200_FIR_TILE=0, profiles/fir_ab.py).  Both stage the x tile (+ tap-chunk
-// halo) and the tap chunk in shared memory, padded so that the sliding-window reads are bank-conflict free.
+// fir_tile_kernel (fir_tile.cuh) evaluates it: a thread owns 8 consecutive outputs (4 for ComplexF64) and walks the taps 8
+// at a time from 128-bit loads, at 62-69 % of the FP32 peak.  The x tile (+ tap-chunk halo) and the tap chunk are staged in
+// shared memory, padded so that the sliding-window reads are bank-conflict free.  It replaced a one-tap-per-iteration kernel
+// on every measured shape (profiles/README.md, FIR table; measured in round 2 with a variant since removed; see the history
+// before this commit).
 #include "common.cuh"
 #include "fir_tile.cuh"
 #include <new>
 
 namespace dspb200 {
 
-template <typename T, bool CPLX> struct fir_elt { using type = T; };
-template <typename T> struct fir_elt<T, true> { using type = cx<T>; };
-
-constexpr int FIR_NT = 256;
-constexpr int FIR_OPT = 4;                      // outputs per thread
-constexpr int FIR_TILE = FIR_NT * FIR_OPT;      // outputs per CTA
-constexpr int FIR_KC = 512;                     // taps per chunk
-
-__host__ __device__ __forceinline__ int fir_pad(int j) { return j + (j >> 5); }
-
-
-template <typename E>
-__global__ void __launch_bounds__(FIR_NT)
-fir_td_kernel(const E* __restrict__ x, int64_t nx, int64_t tiles_per_col, const E* __restrict__ b, int nb,
-              E* __restrict__ out) {
-    __shared__ E xs[FIR_TILE + FIR_KC + (FIR_TILE + FIR_KC) / 32 + 2];
-    __shared__ E bs[FIR_KC];
-    const int tid = threadIdx.x;
-    const int64_t col = blockIdx.x / tiles_per_col;
-    const int64_t tile = blockIdx.x % tiles_per_col;
-    const int64_t i0 = tile * FIR_TILE;
-    const E* xc = x + col * nx;
-    E* oc = out + col * nx;
-    E acc[FIR_OPT];
-#pragma unroll
-    for (int o = 0; o < FIR_OPT; ++o) acc[o] = fir_zero((E*)nullptr);
-
-    // chunks from the oldest taps (largest k) to the newest
-    for (int k_hi = nb - 1; k_hi >= 0; k_hi -= FIR_KC) {
-        const int kc = k_hi + 1 < FIR_KC ? k_hi + 1 : FIR_KC;   // taps k_hi, k_hi-1, .., k_hi-kc+1
-        const int64_t base = i0 - k_hi;                         // global index of xs[0]
-        const int cnt = FIR_TILE + kc - 1;
-        __syncthreads();
-        for (int j = tid; j < cnt; j += FIR_NT) {
-            const int64_t g = base + j;
-            xs[fir_pad(j)] = (g >= 0 && g < nx) ? xc[g] : fir_zero((E*)nullptr);
-        }
-        for (int j = tid; j < kc; j += FIR_NT) bs[j] = b[k_hi - j];
-        __syncthreads();
-        E w[FIR_OPT];
-#pragma unroll
-        for (int o = 0; o < FIR_OPT; ++o) w[o] = xs[fir_pad(FIR_OPT * tid + o)];
-        for (int kk = 0; kk < kc; ++kk) {
-            const E bk = bs[kk];
-#pragma unroll
-            for (int o = 0; o < FIR_OPT; ++o) acc[o] = fir_fma(w[o], bk, acc[o]);
-#pragma unroll
-            for (int o = 0; o < FIR_OPT - 1; ++o) w[o] = w[o + 1];
-            w[FIR_OPT - 1] = xs[fir_pad(FIR_OPT * tid + FIR_OPT + kk)];
-        }
-    }
-#pragma unroll
-    for (int o = 0; o < FIR_OPT; ++o) {
-        const int64_t i = i0 + FIR_OPT * tid + o;
-        if (i < nx) oc[i] = acc[o];
-    }
-}
-
-// ---------------------------------------------------------------------------------------------- register-tiled kernel
 // fir_tile.cuh: a thread owns G consecutive outputs, 8 taps per chunk, two 8-sample register runs that swap roles.
 template <typename E, int NT>
 __global__ void __launch_bounds__(NT)
@@ -156,36 +98,22 @@ int dspb200_fir_exec_dev(dspb200_fir_plan* plan, const void* x, int64_t nx, int6
     if (nx == 0 || ncols == 0) return DSPB200_OK;
     DSP_REQUIRE(x && out, "NULL argument");
     FirPlanImpl* p = &plan->impl;
-    static const bool tiled = [] { const char* e = getenv("DSPB200_FIR_TILE"); return !(e && e[0] == '0'); }();
     cudaStream_t st = (cudaStream_t)stream;
-    if (tiled) {
 #define FIR_TILED(E_) do {                                                                                   \
-            /* short inputs: 128-thread tiles, so that the tiles spread evenly over the SMs */                   \
-            const bool small = cdiv(nx, fir_geom<E_, 256>::TILE) * ncols < (int64_t)8 * device_sm_count();       \
-            const int64_t tiles = cdiv(nx, small ? fir_geom<E_, 128>::TILE : fir_geom<E_, 256>::TILE), blocks = tiles * ncols; \
-            DSP_REQUIRE(blocks < (int64_t)0x7fffffff, "too many tiles for one launch");                          \
-            if (small) fir_tile_kernel<E_, 128><<<(unsigned)blocks, 128, 0, st>>>((const E_*)x, nx, tiles, (const E_*)p->d_b, (int)p->nb, (E_*)out); \
-            else fir_tile_kernel<E_, 256><<<(unsigned)blocks, 256, 0, st>>>((const E_*)x, nx, tiles, (const E_*)p->d_b, (int)p->nb, (E_*)out); \
-        } while (0)
-        switch (p->dtype) {
-            case DSPB200_F32: FIR_TILED(float); break;
-            case DSPB200_F64: FIR_TILED(double); break;
-            case DSPB200_C32: FIR_TILED(cx<float>); break;
-            default: FIR_TILED(cx<double>); break;
-        }
-#undef FIR_TILED
-        DSP_LAUNCH_OK();
-        return DSPB200_OK;
-    }
-    const int64_t tiles = cdiv(nx, FIR_TILE);
-    const int64_t blocks = tiles * ncols;
-    DSP_REQUIRE(blocks < (int64_t)0x7fffffff, "too many tiles for one launch");
+        /* short inputs: 128-thread tiles, so that the tiles spread evenly over the SMs */                   \
+        const bool small = cdiv(nx, fir_geom<E_, 256>::TILE) * ncols < (int64_t)8 * device_sm_count();       \
+        const int64_t tiles = cdiv(nx, small ? fir_geom<E_, 128>::TILE : fir_geom<E_, 256>::TILE), blocks = tiles * ncols; \
+        DSP_REQUIRE(blocks < (int64_t)0x7fffffff, "too many tiles for one launch");                          \
+        if (small) fir_tile_kernel<E_, 128><<<(unsigned)blocks, 128, 0, st>>>((const E_*)x, nx, tiles, (const E_*)p->d_b, (int)p->nb, (E_*)out); \
+        else fir_tile_kernel<E_, 256><<<(unsigned)blocks, 256, 0, st>>>((const E_*)x, nx, tiles, (const E_*)p->d_b, (int)p->nb, (E_*)out); \
+    } while (0)
     switch (p->dtype) {
-        case DSPB200_F32: fir_td_kernel<float><<<(unsigned)blocks, FIR_NT, 0, st>>>((const float*)x, nx, tiles, (const float*)p->d_b, (int)p->nb, (float*)out); break;
-        case DSPB200_F64: fir_td_kernel<double><<<(unsigned)blocks, FIR_NT, 0, st>>>((const double*)x, nx, tiles, (const double*)p->d_b, (int)p->nb, (double*)out); break;
-        case DSPB200_C32: fir_td_kernel<cx<float>><<<(unsigned)blocks, FIR_NT, 0, st>>>((const cx<float>*)x, nx, tiles, (const cx<float>*)p->d_b, (int)p->nb, (cx<float>*)out); break;
-        default: fir_td_kernel<cx<double>><<<(unsigned)blocks, FIR_NT, 0, st>>>((const cx<double>*)x, nx, tiles, (const cx<double>*)p->d_b, (int)p->nb, (cx<double>*)out); break;
+        case DSPB200_F32: FIR_TILED(float); break;
+        case DSPB200_F64: FIR_TILED(double); break;
+        case DSPB200_C32: FIR_TILED(cx<float>); break;
+        default: FIR_TILED(cx<double>); break;
     }
+#undef FIR_TILED
     DSP_LAUNCH_OK();
     return DSPB200_OK;
 }

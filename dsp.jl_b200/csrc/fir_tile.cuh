@@ -4,8 +4,8 @@
 // first.  A thread owns G consecutive outputs and walks the taps eight at a time: the 8 taps of a chunk come from 128-bit
 // broadcast loads, the G + 7 samples those G x 8 products touch are two 8-sample runs in registers; a chunk loads ONE new
 // run (128-bit loads) and the two runs swap roles from chunk to chunk (the loop is unrolled by two: no register shifting).
-// So a Float32 chunk is 4 shared-memory loads + the loop counter for 64 multiply-adds -- the plain kernel (fir_td_kernel)
-// spends two loads and a register shift per 4 multiply-adds and ran at a quarter of the FP32 peak (profiles/r2i_fir.txt).
+// So a Float32 chunk is 4 shared-memory loads + the loop counter for 64 multiply-adds -- the one-tap-per-iteration kernel
+// it replaced spent two loads and a register shift per 4 multiply-adds and ran at a quarter of the FP32 peak (profiles/r2i_fir.txt).
 // The FMA chain of every output is unchanged: bit-identical results.
 //
 // Taps are padded at the OLD end to a multiple of eight; the padding taps are skipped, never multiplied (0 * Inf = NaN):

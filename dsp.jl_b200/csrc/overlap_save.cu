@@ -14,40 +14,8 @@
 #include "async_copy.cuh"
 #include <cufft.h>
 #include <math.h>
-#include <stdlib.h>
 #include <new>
 #include <vector>
-
-// Samples per butterfly of the NEXT unit that are loaded into registers before the current unit's last pass (0 .. 16), so
-// that their L2 -> SM transfer overlaps that pass (timing probes: the exposed first-pass loads are 10 % of the 16384-point
-// kernel).  Measured round 2: the 1024-thread kernel (64 registers per thread) spills 200-1000 bytes with any non-zero
-// value and the 512-thread kernels do not gain, so the shipped library keeps 0 -- the switch stays for tuning.
-#ifndef DSP_OS_PREFETCH
-#define DSP_OS_PREFETCH 0
-#endif
-// threads of the complex 16384-point kernel: 1024 (one butterfly per thread per pass, 64 registers) or 512 (two, 128 registers)
-#ifndef DSP_OS_C16K_THREADS
-#define DSP_OS_C16K_THREADS 1024
-#endif
-// default kernel of the 16384-point Float32 plans: 0 = 16 x 16 x 16 x 4 (fft_core.cuh), 1 = 32 x 32 x 16 (fft_r32.cuh)
-// (measured, 2^26 ComplexF32 samples, 4097 taps: 0.520 ms -> 0.489 ms; real Float32: 0.274 -> 0.269 ms)
-#ifndef DSP_OS_R32_DEFAULT
-#define DSP_OS_R32_DEFAULT 1
-#endif
-// load gating of the 32 x 32 x 16 kernel: bits 0-1 middle passes, bits 2-3 the fused bracket, bits 4-5 the final last pass
-// (measured: 0.489 ms without, 0.504 / 0.519 / 0.517 ms with 3 / 15 / 63 -- two waves of 8 warps do not need it)
-#ifndef DSP_R32_GATE
-#define DSP_R32_GATE 0
-#endif
-// samples (of 32) of the next unit's first-pass butterfly loaded into registers before the current unit's last pass
-// (8 / 16 / 24 all spill 200-350 bytes at 128 registers per thread: the prefetched values end up in local memory; off)
-// request the filter spectrum before the last-pass butterflies of the fused bracket (1) or after them (0)
-#ifndef DSP_R32_HEARLY
-#define DSP_R32_HEARLY 0
-#endif
-#ifndef DSP_R32_PREFETCH
-#define DSP_R32_PREFETCH 0
-#endif
 
 namespace dspb200 {
 
@@ -95,14 +63,14 @@ template <typename T> struct os_elt<T, true> { using type = cx<T>; };
 //  * N = 512 .. 4096 (and the real N = 256 kernel): 1024 resident threads per SM under a 64-register cap, one radix-16
 //    butterfly in flight per thread -- the extra warps hide the shared-memory latency (7-16 % faster than 512 threads
 //    with two butterflies in flight under a 128-register cap);
-//  * complex N = 16384 (one CTA per SM: its shared memory holds one block): 1024 threads, 64-register cap, 9 % faster;
-//  * N = 8192, real N = 16384: 512 resident threads, 128 registers, two butterflies in flight (the 64-register
-//    build spills there and is 2-8 % slower).  Double precision: one CTA of up to 256 registers per thread.
+//  * N = 8192: 512 resident threads, 128 registers, two butterflies in flight (the 64-register build spills there and
+//    is 2-8 % slower).  Double precision: one CTA of up to 256 registers per thread.
+// Float32 N = 16384 runs os_fused32_kernel instead.
 template <typename T, int N, bool CPLX> struct os_threads {
     static constexpr bool f32 = sizeof(T) == 4;
-    static constexpr int value = (f32 && N == 16384 && CPLX) ? DSP_OS_C16K_THREADS : fft_threads<N>::value;
+    static constexpr int value = fft_threads<N>::value;
     static constexpr bool wide = f32 && ((N >= 512 && N <= 4096) || (N == 256 && !CPLX));     // 1024 resident threads
-    static constexpr int minblocks = value == 1024 ? 1 : (wide ? 1024 / value : fft_minblocks<T, N>::value);
+    static constexpr int minblocks = wide ? 1024 / value : fft_minblocks<T, N>::value;
 };
 
 template <typename T> __device__ __forceinline__ cx<T> ldg_cx(const cx<T>* __restrict__ p) {
@@ -137,9 +105,6 @@ __device__ __forceinline__ int os_clamp_diff(int64_t a, int64_t b) {
 // (all units but the first and the last few of a column)
 template <typename T, bool CPLX, bool INTERIOR>
 __device__ __forceinline__ cx<T> os_sample(const OsUnit<typename os_elt<T, CPLX>::type>& g, int j) {
-#if DSP_PROBE & 2
-    return mkc<T>(T(j), T(1));
-#endif
     if constexpr (CPLX) {
         if constexpr (INTERIOR) return g.u[j];
         return (j >= g.jlo && j < g.jhi) ? g.u[j] : mkc<T>(T(0), T(0));
@@ -151,35 +116,35 @@ __device__ __forceinline__ cx<T> os_sample(const OsUnit<typename os_elt<T, CPLX>
         return mkc<T>(a, b);
     }
 }
-// Global loads of a unit's first pass into registers: v[it][r] = sample in slot (tid + it NT) + r N/16, r in [R0, R1).
-template <typename T, int N, bool CPLX, int NT, bool INTERIOR, int ITERS, int R0 = 0, int R1 = 16>
-__device__ __forceinline__ void os_load_unit(const OsUnit<typename os_elt<T, CPLX>::type>& g, int tid, cx<T> (&v)[ITERS][16]) {
-    constexpr int Q = fft_plan_traits<N>::Q;
-#pragma unroll
-    for (int it = 0; it < ITERS; ++it) {
-        const int b = tid + it * NT;
-        if (Q % NT != 0 && b >= Q) break;
-#pragma unroll
-        for (int r = R0; r < R1; ++r) v[it][r] = os_sample<T, CPLX, INTERIOR>(g, b + r * Q);
+
+// Output of slot j of a unit (y: swapped domain, result = (y.y, y.x)); slots below nv-1 produce none.
+template <typename T, bool CPLX, bool INTERIOR>
+__device__ __forceinline__ void os_put(const OsUnit<typename os_elt<T, CPLX>::type>& g, int j, cx<T> y) {
+    if (j < g.nvm1) return;
+    if constexpr (CPLX) {
+        if constexpr (INTERIOR) g.out[j] = mkc<T>(y.y, y.x);
+        else if (j < g.jend) g.out[j] = (j < g.jzero) ? mkc<T>(y.y, y.x) : mkc<T>(T(0), T(0));
+    } else {
+        const int jb = j + g.L;
+        if constexpr (INTERIOR) {
+            g.out[j] = y.y;
+            g.out[jb] = y.x;
+        } else {
+            if (j < g.jend) g.out[j] = (j < g.jzero) ? y.y : T(0);
+            if (jb < g.jend) g.out[jb] = (jb < g.jzero) ? y.x : T(0);
+        }
     }
 }
 
-// One unit.  `vin` holds the unit's samples (os_load_unit); right before the last pass it is refilled with the NEXT unit's
-// samples (next_u: slot 0 of the next unit when that unit is interior, else null): their L2 -> SM transfer (1.4 us per 16384-sample block, ncu / timing probes:
-// 10 % of the kernel when exposed) then overlaps the last pass instead of standing alone at the head of the next unit.
-template <typename T, int N, bool CPLX, int NT, bool INTERIOR, int ITERS>
+// One unit.  The samples are loaded inside the first pass.
+template <typename T, int N, bool CPLX, int NT, bool INTERIOR>
 __device__ __forceinline__ void os_unit(const FftCtx<T>& ctx, int tid, const OsUnit<typename os_elt<T, CPLX>::type>& g,
-                                        const cx<T>* __restrict__ H, cx<T> (&vin)[ITERS][16],
-                                        const typename os_elt<T, CPLX>::type* __restrict__ next_u) {
+                                        const cx<T>* __restrict__ H) {
     constexpr int Q = fft_plan_traits<N>::Q;
-    static_assert(ITERS == (Q + NT - 1) / NT, "register tile does not match the thread count");
+    constexpr int ITERS = (Q + NT - 1) / NT;
     // the barrier inside (between the first butterfly and its stores) also ends the previous unit's last pass
-    if constexpr (DSP_OS_PREFETCH == 0) {
-        auto ld0 = [&](int j, int, int) -> cx<T> { return os_sample<T, CPLX, INTERIOR>(g, j); };
-        fft_first_pass<T, N, NT, true>(ctx, tid, ld0);
-    } else {
-        fft_first_pass_regs<T, N, NT, true>(ctx, tid, vin);
-    }
+    auto ld0 = [&](int j, int, int) -> cx<T> { return os_sample<T, CPLX, INTERIOR>(g, j); };
+    fft_first_pass<T, N, NT, true>(ctx, tid, ld0);
     __syncthreads();
     fft_middle<T, N, NT>(ctx, tid);
     // last forward pass, x H, swap, first pass of the second transform -- in registers
@@ -188,13 +153,9 @@ __device__ __forceinline__ void os_unit(const FftCtx<T>& ctx, int tid, const OsU
     for (int it = 0; it < ITERS; ++it) {
         const int tp = tid + it * NT;
         if (Q % NT == 0 || tp < Q) {
-            fft_last_pass<T, N, (DSP_FFT_GATE && ITERS == 1 && Q % NT == 0) ? NT : 0>(ctx, tp, v[it], tid);
+            fft_last_pass<T, N, (ITERS == 1 && Q % NT == 0) ? NT : 0>(ctx, tp, v[it], tid);
 #pragma unroll
-#if DSP_PROBE & 4
-            for (int r = 0; r < 16; ++r) v[it][r] = cswap(cmul(v[it][r], mkc<T>(T(0.5), T(r))));
-#else
             for (int r = 0; r < 16; ++r) v[it][r] = cswap(cmul(v[it][r], ldg_cx<T>(H + tp + r * Q)));
-#endif
             fft_bfly16_plain<T>(v[it]);
         }
     }
@@ -206,59 +167,25 @@ __device__ __forceinline__ void os_unit(const FftCtx<T>& ctx, int tid, const OsU
     }
     __syncthreads();
     fft_middle<T, N, NT>(ctx, tid);
-    if (next_u != nullptr) {                           // next (interior) unit's samples -> vin, in flight during the last pass
-        OsUnit<typename os_elt<T, CPLX>::type> gn;
-        gn.u = next_u;
-        gn.L = g.L;
-        os_load_unit<T, N, CPLX, NT, true, ITERS, 0, DSP_OS_PREFETCH>(gn, tid, vin);
-    }
+    // Last pass, streamed one radix-RL butterfly at a time: RL live values instead of 16
     constexpr int RL = fft_plan_traits<N>::RL, NBF = 16 / RL;
-    // output of slot j (y: swapped domain, result = (y.y, y.x))
-    auto put = [&](int j, cx<T> y) {
-#if DSP_PROBE & 8
-        if (y.x != T(123456.75)) return;
-#endif
-        if (j < g.nvm1) return;
-        if constexpr (CPLX) {
-            if constexpr (INTERIOR) g.out[j] = mkc<T>(y.y, y.x);
-            else if (j < g.jend) g.out[j] = (j < g.jzero) ? mkc<T>(y.y, y.x) : mkc<T>(T(0), T(0));
-        } else {
-            const int jb = j + g.L;
-            if constexpr (INTERIOR) {
-                g.out[j] = y.y;
-                g.out[jb] = y.x;
-            } else {
-                if (j < g.jend) g.out[j] = (j < g.jzero) ? y.y : T(0);
-                if (jb < g.jend) g.out[jb] = (jb < g.jzero) ? y.x : T(0);
-            }
-        }
+    auto chunk = [&](auto a_, int tp) {
+        constexpr int A = decltype(a_)::value;
+        cx<T> u[RL];
+        fft_last_pass_chunk<T, N, A>(ctx, tp, u);
+#pragma unroll
+        for (int jj = 0; jj < RL; ++jj) os_put<T, CPLX, INTERIOR>(g, tp + (A + NBF * jj) * Q, u[jj]);
     };
-    // Last pass.  The 1024-thread kernel (one butterfly per thread, 64 registers) loads all 16 inputs behind the load gate
-    // and stores 16 outputs (0.531 ms; chunked 0.537); the kernels with two butterflies per thread stream it one radix-RL
-    // butterfly at a time -- RL live values instead of 16 (real 16384-point kernel 0.291 -> 0.271 ms)
-    if constexpr (ITERS == 1 && Q % NT == 0 && NT >= 1024) {
-        fft_last_pass<T, N, DSP_FFT_GATE ? NT : 0>(ctx, tid, v[0], tid);
 #pragma unroll
-        for (int r = 0; r < 16; ++r) put(tid + r * Q, v[0][r]);
-    } else {
-        auto chunk = [&](auto a_, int tp) {
-            constexpr int A = decltype(a_)::value;
-            cx<T> u[RL];
-            fft_last_pass_chunk<T, N, A>(ctx, tp, u);
-#pragma unroll
-            for (int jj = 0; jj < RL; ++jj) put(tp + (A + NBF * jj) * Q, u[jj]);
-        };
-#pragma unroll
-        for (int it = 0; it < ITERS; ++it) {
-            const int tp = tid + it * NT;
-            if (Q % NT != 0 && tp >= Q) break;
-            chunk(std::integral_constant<int, 0>{}, tp);
-            if constexpr (NBF >= 2) chunk(std::integral_constant<int, 1>{}, tp);
-            if constexpr (NBF >= 4) { chunk(std::integral_constant<int, 2>{}, tp); chunk(std::integral_constant<int, 3>{}, tp); }
-            if constexpr (NBF >= 8) {
-                chunk(std::integral_constant<int, 4>{}, tp); chunk(std::integral_constant<int, 5>{}, tp);
-                chunk(std::integral_constant<int, 6>{}, tp); chunk(std::integral_constant<int, 7>{}, tp);
-            }
+    for (int it = 0; it < ITERS; ++it) {
+        const int tp = tid + it * NT;
+        if (Q % NT != 0 && tp >= Q) break;
+        chunk(std::integral_constant<int, 0>{}, tp);
+        if constexpr (NBF >= 2) chunk(std::integral_constant<int, 1>{}, tp);
+        if constexpr (NBF >= 4) { chunk(std::integral_constant<int, 2>{}, tp); chunk(std::integral_constant<int, 3>{}, tp); }
+        if constexpr (NBF >= 8) {
+            chunk(std::integral_constant<int, 4>{}, tp); chunk(std::integral_constant<int, 5>{}, tp);
+            chunk(std::integral_constant<int, 6>{}, tp); chunk(std::integral_constant<int, 7>{}, tp);
         }
     }
 }
@@ -270,8 +197,6 @@ os_fused_kernel(const void* __restrict__ u_, int64_t u_begin, int64_t nu_local, 
                 int64_t zero_from, int nv, int64_t units_per_col, int64_t total_units, const cx<T>* __restrict__ gtl,
                 const cx<T>* __restrict__ g16, const cx<T>* __restrict__ g256, const cx<T>* __restrict__ H) {
     constexpr int NT = os_threads<T, N, CPLX>::value;
-    constexpr int Q = fft_plan_traits<N>::Q;
-    constexpr int ITERS = (Q + NT - 1) / NT;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     cx<T>* sm = reinterpret_cast<cx<T>*>(smem_raw);
     using E = typename os_elt<T, CPLX>::type;
@@ -282,10 +207,8 @@ os_fused_kernel(const void* __restrict__ u_, int64_t u_begin, int64_t nu_local, 
     __syncthreads();
     const int L = N - nv + 1;
     const int span = CPLX ? N : N + L;                 // input samples / output range (+ nv - 1) of one unit
-
-    // geometry of unit gu; returns whether it is interior.  Recomputed where it is needed instead of carried in registers
-    // across the unit (the 1024-thread kernel has 64 registers per thread, 32 of them hold the prefetched samples)
     const bool onecol = units_per_col >= total_units;
+    // geometry of unit gu; returns whether it is interior
     auto geometry = [&](int64_t gu, OsUnit<E>& g) -> bool {
         const int64_t col = onecol ? 0 : gu / units_per_col;
         const int64_t unit = gu - col * units_per_col;
@@ -316,131 +239,57 @@ os_fused_kernel(const void* __restrict__ u_, int64_t u_begin, int64_t nu_local, 
             if (hi > lo && a1 > a0) tma_prefetch_l2(reinterpret_cast<const void*>(a0), (uint32_t)(a1 - a0));
         }
     };
-    // first-pass samples -> vin.  Only INTERIOR units are prefetched across the previous unit's last pass (no predicates,
-    // one base pointer: the 64-register kernel has no room for more); edge units are loaded at the top of their own turn.
-    cx<T> vin[ITERS][16];
-    bool have_vin = false;
-
     for (int64_t gu = blockIdx.x; gu < total_units; gu += gridDim.x) {
-        // while this unit computes, the unit after the next one is pulled into L2; the next one's samples go to registers
-        // right before this unit's last pass (they are L2 hits by then)
-        l2_prefetch(gu + (have_vin ? 2 : 1) * (int64_t)gridDim.x);
+        l2_prefetch(gu + (int64_t)gridDim.x);          // this CTA's next unit, pulled into L2 while this one computes
         OsUnit<E> g;
-        const bool interior = geometry(gu, g);
-        if (DSP_OS_PREFETCH == 0) {
-            // samples are loaded inside the first pass
-        } else if (!have_vin) {
-            if (interior) os_load_unit<T, N, CPLX, NT, true>(g, tid, vin);
-            else os_load_unit<T, N, CPLX, NT, false>(g, tid, vin);
-        } else if (DSP_OS_PREFETCH < 16) {
-            os_load_unit<T, N, CPLX, NT, true, ITERS, DSP_OS_PREFETCH, 16>(g, tid, vin);     // the part that was not prefetched
-        }
-        // the next unit is prefetched by this one iff it is interior
-        const E* next_u = nullptr;
-        {
-            const int64_t gn = gu + gridDim.x;
-            if (gn < total_units) {
-                OsUnit<E> gl;
-                if (geometry(gn, gl)) next_u = gl.u;
-            }
-        }
-        if (DSP_OS_PREFETCH == 0) next_u = nullptr;
-        have_vin = next_u != nullptr;
-        if (interior) os_unit<T, N, CPLX, NT, true>(ctx, tid, g, H, vin, next_u);
-        else os_unit<T, N, CPLX, NT, false>(ctx, tid, g, H, vin, next_u);
+        if (geometry(gu, g)) os_unit<T, N, CPLX, NT, true>(ctx, tid, g, H);
+        else os_unit<T, N, CPLX, NT, false>(ctx, tid, g, H);
     }
 }
 
 // ---------------------------------------------------------------------------------------------- 32 x 32 x 16 kernel
 // The 16384-point Float32 block as 32 x 32 x 16 (fft_r32.cuh): 512 threads, one radix-32 butterfly per thread in the first
 // and the middle pass, two radix-16 butterflies in the last one.  Same unit geometry, same H, same results up to rounding.
-// `pre` / `have_pre`: the first DSP_R32_PREFETCH samples of this thread's first-pass butterfly, loaded by the PREVIOUS unit
-// right before its last pass (next_u: slot 0 of the next unit when that unit is interior, else null) so that part of the
-// L2 -> SM transfer overlaps that pass.
+// It runs every 16384-point Float32 plan (2^26 ComplexF32 samples, 4097 taps: 0.489 ms against 0.520 ms for 16 x 16 x 16 x 4;
+// real Float32: 0.269 against 0.274 ms; measured in round 2 with a variant since removed; see the history before this commit).
 template <typename T, bool CPLX, bool INTERIOR>
 __device__ __forceinline__ void os_unit32(const r32::Ctx<T>& ctx, int tid, const OsUnit<typename os_elt<T, CPLX>::type>& g,
-                                          const cx<T>* __restrict__ H, cx<T> (&pre)[DSP_R32_PREFETCH > 0 ? DSP_R32_PREFETCH : 1],
-                                          bool have_pre, const typename os_elt<T, CPLX>::type* __restrict__ next_u) {
-    constexpr int PF = DSP_R32_PREFETCH;
+                                          const cx<T>* __restrict__ H) {
     cx<T> v[32];
-    if (PF > 0 && have_pre) {
 #pragma unroll
-        for (int r = 0; r < 32; ++r) v[r] = r < PF ? pre[r < PF ? r : 0] : os_sample<T, CPLX, INTERIOR>(g, tid + r * r32::Q32);
-    } else {
-#pragma unroll
-        for (int r = 0; r < 32; ++r) v[r] = os_sample<T, CPLX, INTERIOR>(g, tid + r * r32::Q32);
-    }
+    for (int r = 0; r < 32; ++r) v[r] = os_sample<T, CPLX, INTERIOR>(g, tid + r * r32::Q32);
     fft_bfly<T, 32, true>(v, nullptr);
     __syncthreads();                                   // the previous unit's last pass has read the buffer
     r32::store_block<T>(ctx.sm, tid, v);
     __syncthreads();
-    r32::middle_pass<T, DSP_R32_GATE & 3>(ctx, tid);
+    r32::middle_pass<T>(ctx, tid);
     __syncthreads();
     {
         // last forward pass of the butterflies tid and tid + 512, x H, swap: together they hold Y[tid + 512 m], m < 32,
-        // the inputs of the plain first-pass butterfly of residue class tid of the second transform
+        // the inputs of the plain first-pass butterfly of residue class tid of the second transform.  H is requested
+        // after both butterflies' shared-memory loads.
         cx<T> a[16], b[16];
-#if DSP_R32_HEARLY
-        // H of the first butterfly is requested before its shared-memory loads, H of the second before the second's: the L2
-        // latency of the 32 filter-spectrum loads hides behind the two butterflies instead of following them
-        cx<T> h[16];
-#pragma unroll
-        for (int r = 0; r < 16; ++r) h[r] = ldg_cx<T>(H + tid + r * r32::Q16);
-        r32::last_pass<T>(ctx, tid, a, tid);
-#pragma unroll
-        for (int r = 0; r < 16; ++r) v[2 * r] = cswap(cmul(a[r], h[r]));
-#pragma unroll
-        for (int r = 0; r < 16; ++r) h[r] = ldg_cx<T>(H + tid + r32::Q32 + r * r32::Q16);
-        r32::last_pass<T>(ctx, tid + r32::Q32, b, tid);
-#pragma unroll
-        for (int r = 0; r < 16; ++r) v[2 * r + 1] = cswap(cmul(b[r], h[r]));
-#else
-        r32::last_pass<T, (DSP_R32_GATE >> 2) & 1>(ctx, tid, a, tid);
-        r32::last_pass<T, (DSP_R32_GATE >> 2) & 2>(ctx, tid + r32::Q32, b, tid);
+        r32::last_pass<T>(ctx, tid, a);
+        r32::last_pass<T>(ctx, tid + r32::Q32, b);
 #pragma unroll
         for (int r = 0; r < 16; ++r) {
             v[2 * r] = cswap(cmul(a[r], ldg_cx<T>(H + tid + r * r32::Q16)));
             v[2 * r + 1] = cswap(cmul(b[r], ldg_cx<T>(H + tid + r32::Q32 + r * r32::Q16)));
         }
-#endif
     }
     fft_bfly<T, 32, true>(v, nullptr);
     __syncthreads();                                   // every thread has read its last-pass inputs
     r32::store_block<T>(ctx.sm, tid, v);
     __syncthreads();
-    r32::middle_pass<T, DSP_R32_GATE & 3>(ctx, tid);
+    r32::middle_pass<T>(ctx, tid);
     __syncthreads();
-    if (PF > 0 && next_u != nullptr) {
-        OsUnit<typename os_elt<T, CPLX>::type> gn;
-        gn.u = next_u;
-        gn.L = g.L;
-#pragma unroll
-        for (int r = 0; r < PF; ++r) pre[r] = os_sample<T, CPLX, true>(gn, tid + r * r32::Q32);
-    }
 #pragma unroll
     for (int it = 0; it < 2; ++it) {
         const int tp = tid + it * r32::Q32;
         cx<T> y[16];
-        if (it == 0) r32::last_pass<T, (DSP_R32_GATE >> 4) & 3>(ctx, tp, y, tid);
-        else r32::last_pass<T>(ctx, tp, y);
+        r32::last_pass<T>(ctx, tp, y);
 #pragma unroll
-        for (int r = 0; r < 16; ++r) {
-            const int j = tp + r * r32::Q16;
-            if (j < g.nvm1) continue;
-            if constexpr (CPLX) {                      // swapped domain: result = (y.y, y.x)
-                if constexpr (INTERIOR) g.out[j] = mkc<T>(y[r].y, y[r].x);
-                else if (j < g.jend) g.out[j] = (j < g.jzero) ? mkc<T>(y[r].y, y[r].x) : mkc<T>(T(0), T(0));
-            } else {
-                const int jb = j + g.L;
-                if constexpr (INTERIOR) {
-                    g.out[j] = y[r].y;
-                    g.out[jb] = y[r].x;
-                } else {
-                    if (j < g.jend) g.out[j] = (j < g.jzero) ? y[r].y : T(0);
-                    if (jb < g.jend) g.out[jb] = (jb < g.jzero) ? y[r].x : T(0);
-                }
-            }
-        }
+        for (int r = 0; r < 16; ++r) os_put<T, CPLX, INTERIOR>(g, tp + r * r32::Q16, y[r]);
     }
 }
 
@@ -458,11 +307,11 @@ os_fused32_kernel(const void* __restrict__ u_, int64_t u_begin, int64_t nu_local
     const r32::Ctx<T> ctx = r32::make_ctx<T>(reinterpret_cast<cx<T>*>(smem_raw), g32, g1024, tid);
     pdl_wait();                                        // tables staged; from here on data of preceding kernels is touched
     __syncthreads();
+    // Unit geometry and L2 prefetch as in os_fused_kernel, written out: shared with it as helpers, they changed this
+    // kernel's SASS and cost 0.15 % of the bench conv stage (B200, 1000 W power limit).
     const int L = N - nv + 1;
     const int span = CPLX ? N : N + L;
     const bool onecol = units_per_col >= total_units;
-    cx<T> pre[DSP_R32_PREFETCH > 0 ? DSP_R32_PREFETCH : 1];
-    bool have_pre = false;
     for (int64_t gu = blockIdx.x; gu < total_units; gu += gridDim.x) {
         const int64_t col = onecol ? 0 : gu / units_per_col;
         const int64_t unit = gu - col * units_per_col;
@@ -492,21 +341,8 @@ os_fused32_kernel(const void* __restrict__ u_, int64_t u_begin, int64_t nu_local
             const uintptr_t a1 = (uintptr_t)(reinterpret_cast<const E*>(u_) + coln * u_col_stride + hi) & ~(uintptr_t)15;
             if (hi > lo && a1 > a0) tma_prefetch_l2(reinterpret_cast<const void*>(a0), (uint32_t)(a1 - a0));
         }
-        // the next unit's samples are prefetched by this one iff that unit is interior (same column: slot 0 is L (2L) further)
-        const E* next_u = nullptr;
-        if (DSP_R32_PREFETCH > 0 && gu + gridDim.x < total_units) {
-            const int64_t gn = gu + gridDim.x;
-            const int64_t coln = onecol ? 0 : gn / units_per_col;
-            const int64_t qn = (CPLX ? 1 : 2) * (gn - coln * units_per_col);
-            const int64_t s0n = out_begin + qn * L - (nv - 1);
-            const int64_t i0n = s0n - u_begin;
-            const bool inn = i0n >= 0 && i0n + span <= nu_local && out_begin + out_count - s0n >= span &&
-                             os_clamp_diff(zero_from, s0n) >= span;
-            if (inn) next_u = reinterpret_cast<const E*>(u_) + coln * u_col_stride + i0n;
-        }
-        if (interior) os_unit32<T, CPLX, true>(ctx, tid, g, H, pre, have_pre, next_u);
-        else os_unit32<T, CPLX, false>(ctx, tid, g, H, pre, have_pre, next_u);
-        have_pre = next_u != nullptr;
+        if (interior) os_unit32<T, CPLX, true>(ctx, tid, g, H);
+        else os_unit32<T, CPLX, false>(ctx, tid, g, H);
     }
 }
 
@@ -727,9 +563,7 @@ __global__ void conv_direct_kernel(const void* __restrict__ large_, int64_t nl, 
 }
 
 // ---------------------------------------------------------------------------------------------- dispatch
-#ifndef DSP_OS_SIZES   // (override on the command line to build a single size while tuning)
 #define DSP_OS_SIZES(X) X(32) X(64) X(128) X(256) X(512) X(1024) X(2048) X(4096) X(8192) X(16384)
-#endif
 
 static bool os_fused_ok(int64_t nfft, int64_t nv, bool f64) {
     if (nfft < 32 || (nfft & (nfft - 1))) return false;
@@ -775,13 +609,6 @@ static int launch_os_fused(OsPlanImpl* p, const OsRange& a, cudaStream_t st) {
     return DSPB200_OK;
 }
 
-// which kernel runs a 16384-point Float32 plan: DSPB200_OS_R32 = 0 / 1 forces the 16x16x16x4 / 32x32x16 kernel
-static bool os_use_r32(bool cplx) {
-    if (const char* e = getenv("DSPB200_OS_R32")) return e[0] == '1';
-    (void)cplx;
-    return DSP_OS_R32_DEFAULT != 0;
-}
-
 template <bool CPLX>
 static int launch_os_fused32(OsPlanImpl* p, const OsRange& a, cudaStream_t st) {
     const size_t smem = (size_t)r32::smem_elems<float>() * sizeof(cx<float>);
@@ -803,13 +630,12 @@ static int launch_os_fused32(OsPlanImpl* p, const OsRange& a, cudaStream_t st) {
 
 template <typename T> static int os_fused_dispatch(OsPlanImpl* p, const OsRange& a, cudaStream_t st) {
     if constexpr (sizeof(T) == 4) {
-        if (p->nfft == 16384 && p->d_t32 != nullptr && os_use_r32(p->cplx))
-            return p->cplx ? launch_os_fused32<true>(p, a, st) : launch_os_fused32<false>(p, a, st);
+        if (p->nfft == 16384) return p->cplx ? launch_os_fused32<true>(p, a, st) : launch_os_fused32<false>(p, a, st);
     }
     switch (p->nfft) {
 #define X(NN)                                                                                   \
     case NN:                                                                                    \
-        if constexpr (sizeof(T) == 8 && NN > 8192) break;                                       \
+        if constexpr (NN > 8192) break;      /* Float32: os_fused32_kernel above; Float64 is not fused */ \
         else return p->cplx ? launch_os_fused<T, NN, true>(p, a, st) : launch_os_fused<T, NN, false>(p, a, st);
         DSP_OS_SIZES(X)
 #undef X

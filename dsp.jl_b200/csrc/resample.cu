@@ -11,19 +11,16 @@
 //
 // Layout: CTA = 256 outputs.  The polyphase bank is staged in shared memory phase-major when it fits;
 // x is read through L1/L2 (neighbouring outputs share all but a few samples).
+//
+// rs_launch tries four kernels in order, each covering shapes the previous one cannot: resample_mp2_kernel (pipelined,
+// interp <= 4, decim <= 4, at most 64 taps per phase) -> resample_mp_kernel -> resample_tiled_kernel -> resample_kernel.
+// The pipelined kernel's configuration (4 outputs per phase per thread in Float32, packed FFMA2 for ComplexF32 samples,
+// 128-bit tap loads, the rs_v3 tap rows) is the one that won the resample A/Bs in profiles/README.md; measured in round 2
+// with variants since removed; see the history before this commit.
 #include "common.cuh"
 #include <cuda_pipeline.h>
 #include <new>
 #include <vector>
-
-// outputs per phase per thread of the multi-phase kernel, Float32 arithmetic (register tile)
-#ifndef DSP_RS_G32
-#define DSP_RS_G32 4
-#endif
-
-#ifndef DSP_RS_F32X2
-#define DSP_RS_F32X2 1
-#endif
 
 namespace dspb200 {
 
@@ -38,14 +35,12 @@ template <typename TR> __device__ __forceinline__ TR rs_fma(TR h, TR x, TR acc) 
 template <typename TR> __device__ __forceinline__ cx<TR> rs_fma(TR h, cx<TR> x, cx<TR> acc) {
     return mkc<TR>(fma(h, x.x, acc.x), fma(h, x.y, acc.y));
 }
-#if DSP_RS_F32X2
 // real tap x ComplexF32 sample: both halves in ONE packed FFMA2 (sm_100: two IEEE fused multiply-adds per instruction, the
 // tap broadcast to both halves) -- the same two roundings as the scalar pair, half the issue slots.
 template <> __device__ __forceinline__ cx<float> rs_fma<float>(float h, cx<float> x, cx<float> acc) {
     const float2 r = __ffma2_rn(make_float2(h, h), make_float2(x.x, x.y), make_float2(acc.x, acc.y));
     return mkc<float>(r.x, r.y);
 }
-#endif
 template <typename T> __device__ __forceinline__ T rs_zero(T*) { return T(0); }
 template <typename T> __device__ __forceinline__ cx<T> rs_zero(cx<T>*) { return mkc<T>(T(0), T(0)); }
 
@@ -277,27 +272,21 @@ resample_mp_kernel(const EX* __restrict__ x, int64_t x_begin, int64_t nx_local, 
 //     shared-memory stores (long-scoreboard, 20 % of the samples) is off the critical path;
 //   * two CTA-wide barriers per tile instead of three, no per-tile tap staging.
 // Edge tiles (samples outside the stored range are zero) are filled synchronously with the bounds test.
-#ifndef DSP_RS_HQ
-#define DSP_RS_HQ 1
-#endif
-// DSP_RS_V3 (default): what the ncu capture of the version above (profiles/r2j_resample.txt: FFMA 54 % of the executed
-// instructions although a chunk is 79 % FFMA) showed outside the chunks --
+// The rs_v3 instances also remove what the ncu capture of that version (profiles/r2j_resample.txt: FFMA 54 % of the
+// executed instructions although a chunk is 79 % FFMA) showed outside the chunks --
 //   * the tap rows are staged ONCE per persistent CTA in shared memory and read with 128-bit broadcast loads (6 per chunk
 //     for 3 phases instead of 24 uniform constant loads), which also lets the chunk loop stay ROLLED: two copies of the chunk
 //     body (unchecked, and the checked one for the last chunk's padding taps) instead of eight with a uniform branch per tap
 //     (97 KB of code);
 //   * interior tiles are copied out without the 64-bit bounds tests; single-column launches skip the 64-bit division per tile.
-// Same products in the same order: bit-identical to DSP_RS_V3 = 0 (build target rsv0 for the A/B).
-#ifndef DSP_RS_V3
-#define DSP_RS_V3 1
-#endif
-// V3's tap registers are worth it where the thread's live state (sample window + accumulators + one column group of taps)
+// Same products in the same order as the constant-bank taps: bit-identical.
+// Staged tap rows are worth it where the thread's live state (sample window + accumulators + one column group of taps)
 // still fits the 80-register budget of three resident CTAs and the window addresses are compile-time offsets (8 % GD == 0);
-// the other instances keep the constant-bank taps (they spilled 80-140 bytes with V3).
+// the other instances keep the constant-bank taps (they spilled 80-140 bytes with staged rows).
 template <typename EO, typename TR, int I, int D, int G> struct rs_v3 {
     using M = rs_mp<I, D, G>;
     static constexpr int est = (M::OFFMAX + 8 + M::NO) * (int)(sizeof(EO) / 4) + I * 4;
-    static constexpr bool value = DSP_RS_V3 != 0 && est <= 80 && (8 % M::GD == 0);
+    static constexpr bool value = est <= 80 && (8 % M::GD == 0);
 };
 template <typename TR, int I> struct alignas(16) RsTaps { TR h[I][64]; };
 
@@ -311,7 +300,7 @@ resample_mp2_kernel(const EX* __restrict__ x, int64_t x_begin, int64_t nx_local,
     extern __shared__ __align__(16) unsigned char smem_raw[];
     const int tid = threadIdx.x;
     constexpr bool V3 = rs_v3<EO, TR, I, D, G>::value;
-    TR* hs = reinterpret_cast<TR*>(smem_raw);                                     // V3: [I][64] tap rows, staged once per (persistent) CTA
+    TR* hs = reinterpret_cast<TR*>(smem_raw);                                     // rs_v3: [I][64] tap rows, staged once per (persistent) CTA
     EX* xs0 = reinterpret_cast<EX*>(hs + (V3 ? I * 64 : 0));                      // two skewed sample tiles
     if constexpr (V3) {
         for (int i = tid; i < I * 64; i += M::NTH) {
@@ -394,7 +383,6 @@ resample_mp2_kernel(const EX* __restrict__ x, int64_t x_begin, int64_t nx_local,
 #pragma unroll
         for (int c = 0; c < 8; ++c) {
             if (c < nch) {
-                constexpr int R0 = 0;
                 const int r0 = c * 8;
                 EO xv[M::OFFMAX + 8];
                 if constexpr (8 % M::GD == 0) {
@@ -405,19 +393,12 @@ resample_mp2_kernel(const EX* __restrict__ x, int64_t x_begin, int64_t nx_local,
 #pragma unroll
                     for (int q = 0; q < M::OFFMAX + 8; ++q) xv[q] = rs_cvt<EO, EX>::get(xs[M::xpos(tid * M::GD + r0 + q)]);
                 }
-                TR hq[I][8];                                  // the chunk's taps
-#if DSP_RS_HQ                                                 // 128-bit uniform loads from the parameter bank (A/B: profiles/README.md)
+                TR hq[I][8];                                  // the chunk's taps: 128-bit uniform loads from the parameter bank
 #pragma unroll
                 for (int ph = 0; ph < I; ++ph)
 #pragma unroll
                     for (int v = 0; v < 8; v += 16 / (int)sizeof(TR))
                         *reinterpret_cast<uint4*>(&hq[ph][v]) = *reinterpret_cast<const uint4*>(&taps.h[ph][c * 8 + v]);
-#else                                                         // constant-bank operands of the multiply-adds themselves
-#pragma unroll
-                for (int ph = 0; ph < I; ++ph)
-#pragma unroll
-                    for (int v = 0; v < 8; ++v) hq[ph][v] = taps.h[ph][c * 8 + v];
-#endif
 #pragma unroll
                 for (int q = 0; q < 8; ++q) {
                     if (r0 + q < tpp) {                       // the zero padding taps never touch a sample
@@ -425,7 +406,6 @@ resample_mp2_kernel(const EX* __restrict__ x, int64_t x_begin, int64_t nx_local,
                         for (int o = 0; o < M::NO; ++o) acc[o] = rs_fma(hq[(o * D) % I][q], xv[(o * D) / I + q], acc[o]);
                     }
                 }
-                (void)R0;
             }
         }
         }
@@ -594,16 +574,11 @@ static int rs_launch_mp(RsPlanImpl* p, const RsArgs& a, cudaStream_t st, bool* d
     return DSPB200_OK;
 }
 
-static bool rs_mp2_enabled() {
-    static const bool on = [] { const char* e = getenv("DSPB200_RS_MP2"); return !(e && e[0] == '0'); }();
-    return on;
-}
-
 template <typename EX, typename TR, typename EO, int I, int D, int G>
 static int rs_launch_mp2(RsPlanImpl* p, const RsArgs& a, cudaStream_t st, bool* done) {
     using M = rs_mp<I, D, G>;
     *done = false;
-    if (!rs_mp2_enabled() || p->tpp8 > 64) return DSPB200_OK;
+    if (p->tpp8 > 64) return DSPB200_OK;
     const std::vector<TR>& h8 = [&]() -> const std::vector<TR>& {
         if constexpr (sizeof(TR) == 4) return p->h8_32; else return p->h8_64;
     }();
@@ -649,7 +624,7 @@ static int rs_launch(RsPlanImpl* p, const RsArgs& a, cudaStream_t st) {
     if (p->interp >= 2 && p->interp <= 4 && p->decim <= 4 && p->d_pfb8 && a.phi0 >= 0) {
         // multi-phase kernel: G = outputs per phase per thread (Float32 arithmetic: 4; Float64: 2 -- register budget)
         bool done = false;
-        constexpr int GM = sizeof(TR) == 4 ? DSP_RS_G32 : 2;
+        constexpr int GM = sizeof(TR) == 4 ? 4 : 2;
         const int key = (int)p->interp * 10 + (int)p->decim;
         switch (key) {                                    // pipelined kernel first (taps as kernel parameters, <= 64 per phase)
             case 21: DSP_TRY((rs_launch_mp2<EX, TR, EO, 2, 1, GM>(p, a, st, &done))); break;

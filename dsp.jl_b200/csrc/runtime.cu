@@ -31,10 +31,6 @@ int device_sm_count() {
 }
 
 void count_launch(int n) { g_launches.fetch_add(n, std::memory_order_relaxed); }
-bool pdl_enabled() {
-    static const bool on = [] { const char* e = getenv("DSPB200_PDL"); return !(e && e[0] == '0'); }();
-    return on;
-}
 
 // ---- plan cache / scratch arena of the plan-less entry points
 static std::recursive_mutex g_conv_mutex;

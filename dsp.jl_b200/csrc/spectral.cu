@@ -16,7 +16,6 @@
 #include "async_copy.cuh"
 #include <cufft.h>
 #include <math.h>
-#include <stdlib.h>
 #include <new>
 #include <vector>
 
@@ -68,18 +67,7 @@ struct SpecPlanImpl {
 template <typename T> struct win_t { using type = double; };
 template <> struct win_t<float> { using type = float2; };
 __device__ __forceinline__ double win_mul(double v, double w) { return v * w; }
-// -DDSP_WIN_EXACT=1: the 8 bytes hold the Float64 window value itself and the product is formed exactly as the reference
-// does -- Float32 sample widened, one DMUL, rounded back to Float32 (two conversions + a DMUL on the FP64 pipe per sample).
-#ifndef DSP_WIN_EXACT
-#define DSP_WIN_EXACT 0
-#endif
-#if DSP_WIN_EXACT
-__device__ __forceinline__ float win_mul(float v, float2 w) {
-    return (float)((double)v * __hiloint2double(__float_as_int(w.y), __float_as_int(w.x)));
-}
-#else
 __device__ __forceinline__ float win_mul(float v, float2 w) { return fmaf(v, w.x, v * w.y); }
-#endif
 
 template <typename T, bool CPLX> struct in_type { using type = T; };
 template <typename T> struct in_type<T, true> { using type = cx<T>; };
@@ -838,9 +826,7 @@ __global__ void per2_pad_kernel(const T* __restrict__ s, int64_t n1, int64_t n2,
 }
 
 // ---------------------------------------------------------------------------------------------- dispatch
-#ifndef DSP_FUSED_SIZES   // (override on the command line to build a single size while tuning)
 #define DSP_FUSED_SIZES(X) X(256) X(512) X(1024) X(2048) X(4096) X(8192) X(16384)
-#endif
 
 static bool fused_size_ok(int64_t nfft, bool f64) {
     if (nfft < 256 || (nfft & (nfft - 1))) return false;
@@ -854,7 +840,7 @@ template <typename K> static int set_smem(K kernel, size_t bytes) {
 
 // Launch configuration of the fused Welch kernel: MODE (staging / window placement) x G (thread groups per CTA).  Every
 // candidate that fits is rated by the warps it keeps resident per SM (occupancy calculator x G); ties go to the window
-// in shared memory, then to fewer groups.  DSPB200_WELCH_CFG="mode,groups" forces one (tuning / A-B timing).
+// in shared memory, then to fewer groups.
 template <typename T, int N, bool CPLX>
 static int launch_welch_fused(SpecPlanImpl* p, const void* s, int64_t seg0, int64_t nseg, int64_t sample_offset,
                               cudaStream_t st) {
@@ -869,12 +855,10 @@ static int launch_welch_fused(SpecPlanImpl* p, const void* s, int64_t seg0, int6
     const int64_t units = CPLX ? nseg : (nseg + 1) / 2;
     if (units < 1) return DSPB200_OK;
     const W* win = reinterpret_cast<const W*>(p->d_window);
-    struct Cand { Kern k; size_t smem; int mode, g, warps, per_sm; };
-    Cand best{nullptr, 0, 0, 0, -1, 0};
-    int force_mode = -1, force_g = -1;
-    if (const char* e = getenv("DSPB200_WELCH_CFG")) sscanf(e, "%d,%d", &force_mode, &force_g);
+    struct Cand { Kern k; size_t smem; int g, warps, per_sm; };
+    Cand best{nullptr, 0, 0, -1, 0};
     SpecPlanImpl::WelchCfg& cached = p->welch_cfg[aligned ? 1 : 0];
-    if (cached.kern != nullptr && force_mode < 0 && force_g < 0) {
+    if (cached.kern != nullptr) {
         const int64_t cap = (int64_t)p->sm_count * cached.per_sm;
         const int64_t want = cdiv(units, cached.g);
         const int grid = (int)(want < cap ? want : cap);
@@ -888,10 +872,9 @@ static int launch_welch_fused(SpecPlanImpl* p, const void* s, int64_t seg0, int6
     }
     // candidates are offered in order of preference (measured sweep, profiles/r2_welch_cfg_sweep.jsonl); the first one that
     // keeps at least 12 warps resident per SM is taken, otherwise the one with the most resident warps
-    auto consider = [&](Kern k, size_t smem, int mode, int g) -> int {
-        if (best.warps >= 12 && force_mode < 0) return DSPB200_OK;
+    auto consider = [&](Kern k, size_t smem, int g) -> int {
+        if (best.warps >= 12) return DSPB200_OK;
         if (smem > p->smem_optin) return DSPB200_OK;
-        if ((force_mode >= 0 && mode != force_mode) || (force_g >= 1 && g != force_g)) return DSPB200_OK;
         DSP_TRY(set_smem(k, smem));
         int per_sm = 0;
         DSP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k, NT * g, smem));
@@ -899,12 +882,12 @@ static int launch_welch_fused(SpecPlanImpl* p, const void* s, int64_t seg0, int6
         if ((int64_t)per_sm * g * p->sm_count > p->nparts) per_sm = (int)(p->nparts / ((int64_t)g * p->sm_count));
         if (per_sm < 1) return DSPB200_OK;
         const int warps = per_sm * g * NT / 32;
-        if (warps > best.warps) best = Cand{k, smem, mode, g, warps, per_sm};
+        if (warps > best.warps) best = Cand{k, smem, g, warps, per_sm};
         return DSPB200_OK;
     };
 #define DSP_WELCH_CAND(MODE_, G_)                                                                        \
     DSP_TRY(consider(welch_fused_kernel<T, N, CPLX, MODE_, G_>,                                          \
-                     welch_layout<T, N, CPLX, MODE_>::total(p->n, p->hop, G_), MODE_, G_))
+                     welch_layout<T, N, CPLX, MODE_>::total(p->n, p->hop, G_), G_))
     constexpr bool WREGOK = sizeof(T) == 4 && N <= 4096;           // window in registers: 32 extra registers per thread
     if (aligned) {
         if (win) {
@@ -924,17 +907,12 @@ static int launch_welch_fused(SpecPlanImpl* p, const void* s, int64_t seg0, int6
         DSP_WELCH_CAND(1, 1);
         if constexpr (MULTI) DSP_WELCH_CAND(1, 2);
     }
-    if (best.k == nullptr) {
-        force_mode = force_g = -1;
-        DSP_WELCH_CAND(0, 1);
-    }
+    if (best.k == nullptr) DSP_WELCH_CAND(0, 1);
 #undef DSP_WELCH_CAND
     DSP_REQUIRE(best.k != nullptr, "no Welch kernel configuration fits (nfft=%lld)", (long long)p->nfft);
-    if (force_mode < 0 && force_g < 0) {
-        DSP_TRY(set_smem(best.k, best.smem));          // (the last candidate examined may have left a different limit)
-        cached.kern = reinterpret_cast<void*>(best.k); cached.smem = best.smem; cached.g = best.g; cached.per_sm = best.per_sm;
-        cached.threads = NT * best.g;
-    }
+    DSP_TRY(set_smem(best.k, best.smem));              // (the last candidate examined may have left a different limit)
+    cached.kern = reinterpret_cast<void*>(best.k); cached.smem = best.smem; cached.g = best.g; cached.per_sm = best.per_sm;
+    cached.threads = NT * best.g;
     // one wave of persistent CTAs: exactly the number that is co-resident; (CTAs x groups) never exceeds the rows of `partial`
     const int64_t cap = (int64_t)p->sm_count * best.per_sm;
     const int64_t want = cdiv(units, best.g);
@@ -974,11 +952,10 @@ static int launch_stft_fused(SpecPlanImpl* p, const void* s, int64_t len, int64_
     if (units < 1) return DSPB200_OK;
     const auto* w = reinterpret_cast<const typename win_t<T>::type*>(p->d_window);
     if constexpr (sizeof(T) == 4 && N == 1024) {
-        // one warp per unit (stft_w1k_kernel): needs the TMA alignment conditions; DSPB200_STFT_W1K=0 forces the CTA kernel
-        const char* e = getenv("DSPB200_STFT_W1K");
+        // one warp per unit (stft_w1k_kernel): needs the TMA alignment conditions
         const bool aligned = ((uintptr_t)s % 16 == 0) && ((len * sizeof(In)) % 16 == 0 || nchan == 1) &&
                              ((p->hop * sizeof(In)) % 16 == 0) && ((p->n * sizeof(In)) % 16 == 0);
-        if (aligned && p->d_t32 != nullptr && !(e && e[0] == '0')) {
+        if (aligned && p->d_t32 != nullptr) {
             constexpr int WARPS = 4;
             const size_t smem1 = (size_t)w1k::T32_LEN * sizeof(cx<float>) + (w ? (size_t)p->n * sizeof(float2) : 0) +
                                  (size_t)WARPS * w1k::warp_bytes(CPLX ? p->n : p->hop + p->n, sizeof(In));
@@ -1334,8 +1311,6 @@ static int spec_plan_create_impl(dspb200_spec_plan** plan, int dtype, int64_t n,
             cudaError_t e = cudaMalloc(&p->d_window, (size_t)nw * sizeof(double));
             if (e == cudaSuccess) {
                 if (p->f64) {
-                    e = cudaMemcpy(p->d_window, window_host, (size_t)nw * sizeof(double), cudaMemcpyHostToDevice);
-                } else if (DSP_WIN_EXACT) {                 // the Float64 values themselves (win_mul widens the sample)
                     e = cudaMemcpy(p->d_window, window_host, (size_t)nw * sizeof(double), cudaMemcpyHostToDevice);
                 } else {                                   // hi/lo float pairs (same 8 bytes per value)
                     std::vector<float> pairs((size_t)nw * 2);

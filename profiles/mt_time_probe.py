@@ -1,4 +1,4 @@
-"""Where does the host-array spectrogram spend its time (plan creation / exec / close)?  DSPB200_STFT_W1K=0|1."""
+"""Where does the host-array spectrogram spend its time (plan creation / exec / close)?"""
 import os
 import sys
 import time
@@ -27,4 +27,4 @@ for rep in range(4):
     t3 = time.perf_counter()
     plan.close()
     t4 = time.perf_counter()
-    print(f"W1K={os.environ.get('DSPB200_STFT_W1K')} create {1e3 * (t1 - t0):.2f} ms, exec#1 {1e3 * (t2 - t1):.2f}, exec#2 {1e3 * (t3 - t2):.2f}, close {1e3 * (t4 - t3):.2f}")
+    print(f"create {1e3 * (t1 - t0):.2f} ms, exec#1 {1e3 * (t2 - t1):.2f}, exec#2 {1e3 * (t3 - t2):.2f}, close {1e3 * (t4 - t3):.2f}")

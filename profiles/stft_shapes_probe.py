@@ -1,5 +1,5 @@
 """Kernel-only timing of the fused STFT (nfft = 1024, Float32) over a few shapes: channels x length, hop, window.
-    python profiles/stft_shapes_probe.py      (DSPB200_STFT_W1K=0 selects the CTA kernel)"""
+    python profiles/stft_shapes_probe.py"""
 import os
 import sys
 
@@ -36,5 +36,5 @@ for nchan, log2len, nov, usewin in ((64, 22, 768, False), (64, 22, 768, True), (
     k = plan.nsegments(length)
     out = torch.empty(513 * k * nchan, device=dev)
     ms = timeit(lambda: plan.stft_dev(x.data_ptr(), length, nchan, 1024.0, True, out.data_ptr(), 0))
-    print(f"nchan={nchan:3d} len=2^{log2len} noverlap={nov} window={usewin}: {ms:.4f} ms  ({nchan * length / ms / 1e6:.1f} Gsamples/s)  W1K={os.environ.get('DSPB200_STFT_W1K')}")
+    print(f"nchan={nchan:3d} len=2^{log2len} noverlap={nov} window={usewin}: {ms:.4f} ms  ({nchan * length / ms / 1e6:.1f} Gsamples/s)")
     del x, out
